@@ -27,6 +27,8 @@ region of >= 10 s (SURVEY §8d "steady state, >= 10 s").
           each channel's (burst, idx, frame octets, FEC corrections, header syndrome weight) list and counters and
           compares them with the oracle (run as a separate checker process on the 64 slot channels); a mismatch
           anywhere makes the benchmark fail.
+  --dump-outputs DIR : after the timed legs, what the timed device path delivered for its last step is written to DIR as
+          .npy files (see dump_outputs); the inputs depend on the arguments only, so two builds compare output for output.
   --impl reference : the unmodified reference (oracle/_ref/vdl2_ref_fast, one pinned pthread per channel, all host
           threads) on a bounded sample of the same stream; falls back to the oracle port if _ref is absent.
 """
@@ -54,6 +56,10 @@ N_SLOTS = 64
 B_CS = 8.0 + 8.0 / OVERSAMPLE        # algorithmic bytes per channel-sample for K1 (SURVEY.md §8d): 8 B read + 8/os B written
 PARITY_CHUNKS = 8                    # the first second of the stream is re-run for the in-bench parity check
 METRIC = "VDL2 channel-samples demodulated per second (2.1 Msps channels; real-time channels = value/2.1)"
+DUMP_CHANNELS = 512                  # --dump-outputs: fixed, seeded sample of channels whose frames are written
+DUMP_BYTES = 64 << 20                # --dump-outputs: cap on all files together
+FRAME_FIELDS = ["channel", "burst_seq", "idx", "len", "synd_weight", "datalen_octets", "num_fec_corrections", "fcs_ok",
+                "sync_dec_index", "frame_pwr_dbfs", "nf_pwr_dbfs", "ppm_error", "frame_pwr", "mag_nf"]
 
 
 def make_stream(seconds):
@@ -219,6 +225,36 @@ def run_reference(args, rank):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, frames, counters, first_dec, suffix=""):
+    """--dump-outputs: the frames the timed device path delivered for its last step and the per-channel counters after it.
+
+    frames_meta.npy      float64 [n, len(FRAME_FIELDS)]: one row per frame, columns FRAME_FIELDS (every value exact)
+    frames_data.npy      float32 [sum of len]: the frames' octets back to back, in row order
+    frames_channels.npy  float64: the sampled channels, sorted
+    channel_counters.npy float64 [channels, 9]: api.COUNTER_NAMES per channel, cumulative over the whole leg
+    Frames are those synced in the last step (sync_dec_index >= first_dec: which poll of the pipeline hands over a frame
+    near a step boundary depends on timing, where its burst was synced does not) on a fixed, seeded sample of
+    DUMP_CHANNELS channels, sorted by (channel, burst, idx) and cut where the files would exceed DUMP_BYTES."""
+    n_ch = counters.shape[0]
+    sample = np.sort(np.random.default_rng(0x56444C33).choice(n_ch, min(DUMP_CHANNELS, n_ch), replace=False))
+    keep = set(int(c) for c in sample)
+    budget = DUMP_BYTES - counters.size * 8 - sample.size * 8
+    rows, data = [], []
+    for f in sorted((f for f in frames if f.channel in keep and f.sync_dec_index >= first_dec), key=lambda f: f.key()):
+        budget -= len(FRAME_FIELDS) * 8 + len(f.data) * 4
+        if budget < 0:
+            break
+        rows.append([float(getattr(f, k)) if k != "len" else float(len(f.data)) for k in FRAME_FIELDS])
+        data.append(np.frombuffer(f.data, np.uint8))
+    os.makedirs(out_dir, exist_ok=True)
+    meta = np.array(rows, np.float64).reshape(-1, len(FRAME_FIELDS))
+    np.save(os.path.join(out_dir, f"frames_meta{suffix}.npy"), meta)
+    np.save(os.path.join(out_dir, f"frames_data{suffix}.npy"), (np.concatenate(data) if data else np.zeros(0, np.uint8)).astype(np.float32))
+    np.save(os.path.join(out_dir, f"frames_channels{suffix}.npy"), sample.astype(np.float64))
+    np.save(os.path.join(out_dir, f"channel_counters{suffix}.npy"), counters.astype(np.float64))
+    print(f"--dump-outputs: {meta.shape[0]} frames of {sample.size} channels, counters of {n_ch} channels -> {out_dir}", file=sys.stderr)
+
+
 # ------------------------------------------------------------------------------------------------------------------
 # parity checker (the oracle runs in its own process: nothing under oracle/ is loaded into the measured process)
 # ------------------------------------------------------------------------------------------------------------------
@@ -275,6 +311,7 @@ def main():
     ap.add_argument("--no-repeat", action="store_true", help="skip the second value/e2e pair and the other channel order")
     ap.add_argument("--k1-scalar", action="store_true")
     ap.add_argument("--fanout", default="nccl", choices=["auto", "nccl", "ce"], help="multi-GPU ingest: NCCL broadcast (default) or copy-engine peer copies")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last step to DIR/*.npy")
     ap.add_argument("--oracle-digest", nargs=2, metavar=("IN", "OUT"), help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.oracle_digest:
@@ -352,7 +389,7 @@ def main():
             k = j + 1
         return runs
 
-    def step_multi(src_rows, src_is_host):
+    def step_multi(src_rows, src_is_host, harvest=True):
         """stage step s+1 (rank 0 gathers the chunks into the free half of the receive area, all ranks take part in the
         fan-out) BEFORE the chunks of step s are submitted: the transfer overlaps the kernels.  A staged step is always
         consumed, also across the legs of the benchmark (its bytes are the same whichever memory they came from)."""
@@ -363,31 +400,33 @@ def main():
         t0 = time.perf_counter()
         mg.submit_staged(buf, CPS, CHUNK_BYTES)
         host_t["submit_s"] += time.perf_counter() - t0; host_t["submits"] += CPS
-        return g.poll_count()
+        return g.poll_count() if harvest else 0
 
-    def step_device():
+    def step_device(harvest=True):
         """one step, chunks already in HBM (N>1: fanned out from rank 0, one step ahead)"""
         if world > 1:
-            return step_multi(d_chunks if rank == 0 else None, False)
+            return step_multi(d_chunks if rank == 0 else None, False, harvest)
         t0 = time.perf_counter()
         for i in next_indices():
             g.submit_device(d_chunks[i].data_ptr(), CHUNK_BYTES, stream.cuda_stream)
         host_t["submit_s"] += time.perf_counter() - t0; host_t["submits"] += CPS
-        return g.poll_count()
+        return g.poll_count() if harvest else 0
 
-    def step_host():
+    def step_host(harvest=True):
         """one step through the public host-buffer entry point (process_buf_uchar); with N > 1 the ingest rank copies
         the step's chunks host->device and fans them out, the other ranks receive"""
         if world > 1:
-            return step_multi(h_chunks, True)
+            return step_multi(h_chunks, True, harvest)
         hn = h_chunks.numpy()
         t0 = time.perf_counter()
         for i in next_indices():
             g.process_buf_uchar(hn[i])
         host_t["submit_s"] += time.perf_counter() - t0; host_t["submits"] += CPS
-        return g.poll_count()
+        return g.poll_count() if harvest else 0
 
-    def timed(step_fn, steps, sample_clocks=False):
+    def timed(step_fn, steps, sample_clocks=False, capture=False):
+        """capture: the last step's frames are not harvested inside the timed region; the region ends when the device has
+        drained, and they are collected after it (r["captured"])"""
         sampler = ClockSampler(local_rank) if (sample_clocks and rank == 0) else None
         barrier()
         s0 = g.stats()
@@ -400,14 +439,20 @@ def main():
         ev[0].record(stream)
         frames = 0
         for k in range(steps):
-            frames += step_fn()          # submits + non-blocking harvest: the pipeline stays full across steps
+            frames += step_fn(not (capture and k == steps - 1))     # submits + non-blocking harvest: the pipeline stays full across steps
             g.stream_wait(stream.cuda_stream)
             ev[k + 1].record(stream)     # completes when every kernel of steps 0..k has run
-        frames += g.flush_count()        # everything submitted is processed and its frames are on the host
+        if not capture:
+            frames += g.flush_count()    # everything submitted is processed and its frames are on the host
         g.stream_wait(stream.cuda_stream)
         ev[steps + 1].record(stream)
         barrier()
         t1 = time.time()
+        captured = None
+        if capture:
+            captured = dict(frames=g.flush(), counters=g.channel_counters(),
+                            first_dec=(s0["iq_samples"] + (steps - 1) * CPS * CHUNK_PAIRS) // OVERSAMPLE + 1)
+            frames += len(captured["frames"])
         ms = ev[0].elapsed_time(ev[steps + 1])
         per = [ev[k].elapsed_time(ev[k + 1]) for k in range(steps)]
         if world > 1:
@@ -417,14 +462,14 @@ def main():
         clocks = sampler.stop(t0, t1) if sampler else None
         s1 = g.stats()
         return dict(ms=ms, per_step=per, frames=frames, d={k: s1[k] - s0[k] for k in s1}, clocks=clocks, wall_ms=(t1 - t0) * 1e3,
-                    host_us_per_submit=host_t["submit_s"] / max(host_t["submits"], 1) * 1e6)
+                    host_us_per_submit=host_t["submit_s"] / max(host_t["submits"], 1) * 1e6, captured=captured)
 
-    def leg(kind, steps, warm, sample_clocks=False):
+    def leg(kind, steps, warm, sample_clocks=False, capture=False):
         fn = step_device if kind == "device" else step_host
         for _ in range(warm):
             fn()
         g.flush_count()
-        r = timed(fn, steps, sample_clocks)
+        r = timed(fn, steps, sample_clocks, capture)
         g.flush_count()
         return r
 
@@ -434,7 +479,11 @@ def main():
         return cs_per_step * steps / (r["ms"] * 1e-3) / 1e6
 
     # ---- A-B-A-B ----
-    A1 = leg("device", K, W, sample_clocks=True)
+    A1 = leg("device", K, W, sample_clocks=True, capture=bool(args.dump_outputs))
+    if args.dump_outputs:
+        cap = A1.pop("captured")
+        dump_outputs(args.dump_outputs, cap["frames"], cap["counters"], cap["first_dec"], f"_rank{rank}" if world > 1 else "")
+        del cap
     B1 = leg("host", K, 1)
     A2 = B2 = None
     if not args.no_repeat:

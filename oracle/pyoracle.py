@@ -32,16 +32,13 @@ class VoEvent(C.Structure):
 
 
 def build(force=False):
-    """(Re)build liboracle.so and, when /root/reference is present, oracle/_ref."""
+    """(Re)build liboracle.so and, when the reference sources are present (REF in oracle/Makefile), oracle/_ref."""
     so = os.path.join(_HERE, "liboracle.so")
     src = [os.path.join(_HERE, f) for f in ("vdl2_oracle.c", "vdl2_oracle.h")]
     stale = force or not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src)
     if stale:
         subprocess.check_call(["make", "-C", _HERE, "liboracle.so"], stdout=subprocess.DEVNULL)
-    if os.path.isdir("/root/reference/src"):
-        subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)
-        if os.path.exists(os.path.join(_HERE, "..", "dumpvdl2_b200", "libvdl2gpu.so")):
-            subprocess.check_call(["make", "-C", _HERE, "dropin"], stdout=subprocess.DEVNULL)
+    subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)
     return so
 
 

@@ -212,5 +212,43 @@ def case_replicas(n_slots=16, n_rep=4, duration=0.5, seed=0x56444C33, es_n0_db=2
     return _mk(f"replicas_{n_slots}x{n_rep}", fs, "u8", freqs, iq, chunk=524288, bursts=bursts)
 
 
+def case_fuzz():
+    """Differential fuzz of the burst decoder: transmissions whose payloads are random bits, or stuffed frames cut at a
+    random bit, some with corrupted code words and header bits, on two channels."""
+    rng = np.random.default_rng(0x7E7E)
+    F = "01111110"
+
+    def stuffed(n):
+        return "".join(format(b, "08b")[::-1] for b in rng.integers(0, 256, n, dtype=np.uint8)).replace("11111", "111110")
+    fs, offs = 2100000, [100e3, -100e3]
+    bursts, t = [], [0.02, 0.02]
+    for k in range(18):
+        nbits = int(rng.integers(40, 5000))
+        if k % 3 == 0:
+            pl = "".join("01"[b] for b in rng.integers(0, 2, nbits, dtype=np.uint8))
+        else:
+            pl = F
+            while len(pl) < nbits:
+                pl += stuffed(int(rng.integers(0, 200))) + F * int(rng.integers(1, 3))
+            if k % 3 == 1:
+                pl = pl[:nbits]
+        n_oct = -(-len(pl) // 8)
+        nblk = -(-n_oct // 249)
+        corrupt = [(int(rng.integers(0, nblk)), int(rng.integers(0, min(249, n_oct - (nblk - 1) * 249))), int(rng.integers(1, 256)))
+                   for _ in range(int(rng.integers(0, 5)) if k % 2 else 0)]
+        hdr = (int(rng.integers(0, 25)),) if k % 5 == 4 else ()
+        ch = k % 2
+        try:
+            synth.burst_bits_from_payload(pl, corrupt)
+        except ValueError:
+            continue
+        bursts.append(synth.BurstSpec(t[ch], offs[ch], [], power_dbfs=-12.0, payload=pl, corrupt_octets=corrupt, header_bit_errors=hdr))
+        t[ch] += synth.burst_duration_s(None, payload=pl) + 0.012
+    iq = synth.synth_stream(fs, max(t) + 0.02, bursts, es_n0_db=32, fmt="u8", seed=0x7E7F)
+    return _mk("fuzz", fs, "u8", [CENTER + o for o in offs], iq, chunk=524288, bursts=bursts)
+
+
 ALL_GOLDEN = {"wav": case_wav, "cfg2": case_cfg2, "mixed_s16": case_mixed_s16, "fec": case_fec, "noisy": case_noisy,
               "hdlc_edge": case_hdlc_edge, "mirics_os13": case_mirics_os13, "maxlen": case_maxlen}
+# streams whose reference output is stored too, but which only the CPU oracle is compared with (test_oracle.py)
+ORACLE_GOLDEN = {"replicas_8x2": lambda: case_replicas(n_slots=8, n_rep=2, duration=0.4), "stress": case_stress, "fuzz": case_fuzz}

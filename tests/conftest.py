@@ -12,7 +12,7 @@ def pytest_configure(config):
 
 def pytest_sessionstart(session):
     """Make sure the native pieces exist before any test imports them: libvdl2gpu.so (nvcc cross-compiles without
-    a GPU), the oracle and - where /root/reference is mounted - oracle/_ref and the drop-in harness."""
+    a GPU) and the oracle."""
     try:
         from dumpvdl2_b200.build import build_native
         build_native()

@@ -1,10 +1,7 @@
-"""CPU: the oracle restatement against (a) the reference's own fixture and the outputs of the unmodified
-reference stored in tests/golden (made by tests/golden/make_golden.py), (b) the live oracle/_ref binaries
-when they are present, (c) the reference's table literals when /root/reference is mounted."""
+"""CPU: the oracle restatement against the reference's own fixture and against what the unmodified reference
+produced, stored in tests/golden by tests/golden/make_golden.py: its output on the streams of tests/cases.py and
+its table literals."""
 import hashlib
-import os
-import re
-import tempfile
 import numpy as np
 import pytest
 from oracle import pyoracle as po
@@ -50,89 +47,52 @@ def test_injected_frames_come_back():
     assert want <= got and len(want) == 12
 
 
-@pytest.mark.skipif(po.ref_binary("strict") is None, reason="oracle/_ref not built (needs /root/reference)")
+def _oracle_and_reference(name, flavour):
+    """the oracle's frames on a stored stream (sorted by key) and the reference's output on it (tests/golden, per
+    channel in push order)"""
+    c = cases.ORACLE_GOLDEN[name]()
+    gold = util.load_golden(name)
+    assert cases.iq_sha256(c) == gold["iq_sha256"], "stream regenerated from the seed differs from the golden's"
+    return sorted(util.run_oracle(c).frames(), key=lambda f: f.key()), gold[flavour]
+
+
 @pytest.mark.parametrize("flavour", ["strict", "fast"])
 def test_oracle_matches_live_reference_on_replicas(flavour):
-    c = cases.case_replicas(n_slots=8, n_rep=2, duration=0.4)
-    with tempfile.NamedTemporaryFile(suffix=".cu8") as tf:
-        tf.write(c["iq"].tobytes()); tf.flush()
-        ref, _ = po.run_ref(tf.name, po.FMT_U8, c["oversample"], c["centerfreq"], c["freqs"], flavour=flavour, chunk=c["chunk"])
-    fr = sorted(util.run_oracle(c).frames(), key=lambda f: f.key())
+    fr, ref = _oracle_and_reference("replicas_8x2", flavour)
     assert len(fr) == len(ref) and len(fr) > 4
     for a, b in zip(fr, ref):
-        assert (a.channel, a.idx, a.data) == (b["channel"], b["idx"], b["data"])
+        assert (a.channel, a.idx, a.data.hex()) == (b["channel"], b["idx"], b["hex"])
         if flavour == "strict":     # the -ffast-math build may slice a marginal symbol differently (RS then repairs it)
             assert a.num_fec_corrections == b["num_fec_corrections"]
 
 
-@pytest.mark.skipif(po.ref_binary("strict") is None, reason="oracle/_ref not built (needs /root/reference)")
 def test_oracle_matches_live_reference_on_stress_stream():
     """Demodulator-side differential: carrier offsets, clipping / very weak bursts, back-to-back and overlapping
     bursts (cases.case_stress) - frames and printed metadata identical to the strictly compiled reference."""
-    c = cases.case_stress()
-    with tempfile.NamedTemporaryFile(suffix=".cu8") as tf:
-        tf.write(c["iq"].tobytes()); tf.flush()
-        ref, _ = po.run_ref(tf.name, po.FMT_U8, c["oversample"], c["centerfreq"], c["freqs"], flavour="strict", chunk=c["chunk"])
-    fr = sorted(util.run_oracle(c).frames(), key=lambda f: f.key())
+    fr, ref = _oracle_and_reference("stress", "strict")
     assert len(fr) == len(ref) and len(fr) > 15, (len(fr), len(ref))
     for a, b in zip(fr, ref):
-        assert (a.channel, a.idx, a.data, a.num_fec_corrections, a.synd_weight) == (b["channel"], b["idx"], b["data"], b["num_fec_corrections"], b["synd_weight"])
+        assert (a.channel, a.idx, a.data.hex(), a.num_fec_corrections, a.synd_weight) == (b["channel"], b["idx"], b["hex"], b["num_fec_corrections"], b["synd_weight"])
         assert abs(a.frame_pwr_dbfs - b["frame_pwr_dbfs"]) < 2e-3 and abs(a.nf_pwr_dbfs - b["nf_pwr_dbfs"]) < 2e-3
         assert abs(a.ppm_error - b["ppm_error"]) < 2e-3
 
 
-@pytest.mark.skipif(po.ref_binary("strict") is None, reason="oracle/_ref not built (needs /root/reference)")
 def test_oracle_matches_live_reference_on_fuzzed_payloads():
-    """Differential fuzz of the burst decoder against the reference itself: transmissions whose payloads are random
-    bits, or stuffed frames cut at a random bit, some with corrupted code words and header bits, modulated and run
-    through oracle/_ref (unmodified src/decode.c, bitstream.c, rs.c) and through the restatement."""
-    from dumpvdl2_b200 import synth
-    rng = np.random.default_rng(0x7E7E)
-    F = "01111110"
-
-    def stuffed(n):
-        return "".join(format(b, "08b")[::-1] for b in rng.integers(0, 256, n, dtype=np.uint8)).replace("11111", "111110")
-    fs, offs = 2100000, [100e3, -100e3]
-    bursts, t = [], [0.02, 0.02]
-    for k in range(18):
-        nbits = int(rng.integers(40, 5000))
-        if k % 3 == 0:
-            pl = "".join("01"[b] for b in rng.integers(0, 2, nbits, dtype=np.uint8))
-        else:
-            pl = F
-            while len(pl) < nbits:
-                pl += stuffed(int(rng.integers(0, 200))) + F * int(rng.integers(1, 3))
-            if k % 3 == 1:
-                pl = pl[:nbits]
-        n_oct = -(-len(pl) // 8)
-        nblk = -(-n_oct // 249)
-        corrupt = [(int(rng.integers(0, nblk)), int(rng.integers(0, min(249, n_oct - (nblk - 1) * 249))), int(rng.integers(1, 256)))
-                   for _ in range(int(rng.integers(0, 5)) if k % 2 else 0)]
-        hdr = (int(rng.integers(0, 25)),) if k % 5 == 4 else ()
-        ch = k % 2
-        try:
-            synth.burst_bits_from_payload(pl, corrupt)
-        except ValueError:
-            continue
-        bursts.append(synth.BurstSpec(t[ch], offs[ch], [], power_dbfs=-12.0, payload=pl, corrupt_octets=corrupt, header_bit_errors=hdr))
-        t[ch] += synth.burst_duration_s(None, payload=pl) + 0.012
-    iq = synth.synth_stream(fs, max(t) + 0.02, bursts, es_n0_db=32, fmt="u8", seed=0x7E7F)
-    c = cases._mk("fuzz", fs, "u8", [cases.CENTER + o for o in offs], iq, chunk=524288, bursts=bursts)
-    with tempfile.NamedTemporaryFile(suffix=".cu8") as tf:
-        tf.write(c["iq"].tobytes()); tf.flush()
-        ref, _ = po.run_ref(tf.name, po.FMT_U8, c["oversample"], c["centerfreq"], c["freqs"], flavour="strict", chunk=c["chunk"])
-    fr = sorted(util.run_oracle(c).frames(), key=lambda f: f.key())
+    """Differential fuzz of the burst decoder against the reference itself (cases.case_fuzz): random-bit payloads and
+    stuffed frames cut at a random bit, some with corrupted code words and header bits, decoded by the unmodified
+    src/decode.c, bitstream.c, rs.c and by the restatement."""
+    fr, ref = _oracle_and_reference("fuzz", "strict")
     assert len(fr) == len(ref) and len(fr) > 20
     for a, b in zip(fr, ref):
-        assert (a.channel, a.idx, a.data, a.num_fec_corrections, a.synd_weight) == (b["channel"], b["idx"], b["data"], b["num_fec_corrections"], b["synd_weight"])
+        assert (a.channel, a.idx, a.data.hex(), a.num_fec_corrections, a.synd_weight) == (b["channel"], b["idx"], b["hex"], b["num_fec_corrections"], b["synd_weight"])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference sources not mounted")
 def test_tables_against_reference_literals():
-    src = open("/root/reference/src/decode.c").read()
-    rows = [int(x, 2) for x in re.findall(r"0b([01]{25})", src.split("syndtable")[0])]
-    pats = [int(x, 2) for x in re.findall(r"0b([01]{25})", src.split("syndtable")[1].split("synd_weight")[0])]
-    weights = [int(x) for x in re.findall(r"\d+", src.split("synd_weight[1<<HDRFECLEN] = {")[1].split("}")[0])]
+    """header syndrome weights and error patterns (src/decode.c) and the CRC-16 table (src/crc.c), as stored from the
+    reference's literals in tests/golden/ref_tables.json"""
+    t = util.load_golden("ref_tables")
+    pats, weights, crc_tab = t["syndrome_patterns"], t["synd_weight"], t["crc16_table"]
+    assert len(t["syndrome_rows"]) == 5 and len(pats) == 32 and len(weights) == 32 and len(crc_tab) == 256
     import ctypes as C
     L = po.lib()
     for syn in range(32):
@@ -146,8 +106,6 @@ def test_tables_against_reference_literals():
         w = C.c_uint32(pat)
         s = L.vo_header_decode(C.byref(w))
         assert w.value == 0 and pats[s] == pat
-    assert len(rows) == 5
-    crc_tab = [int(x, 16) for x in re.findall(r"0x([0-9A-F]{4})", open("/root/reference/src/crc.c").read().split("crctable[256]")[1])][:256]
     for b in range(256):
         assert po.crc16(bytes([b]), init=0) == crc_tab[b]
 
