@@ -35,6 +35,10 @@ class _Config(C.Structure):
                 ("flags", C.c_uint32), ("n_inflight", C.c_uint32), ("n_streams", C.c_uint32), ("reserved", C.c_uint32 * 4)]
 
 
+class _StreamLayout(C.Structure):
+    _fields_ = [("n_streams", C.c_uint32), ("channels_per_stream", C.POINTER(C.c_uint32)), ("centerfreqs", C.POINTER(C.c_uint32))]
+
+
 class _Frame(C.Structure):
     _fields_ = [("channel", C.c_uint32), ("freq", C.c_uint32), ("burst_seq", C.c_uint32), ("idx", C.c_int32),
                 ("data", C.POINTER(C.c_uint8)), ("len", C.c_uint32), ("synd_weight", C.c_uint32),
@@ -70,6 +74,7 @@ def load_library():
                            "(nvcc, sm_100a). There is no CPU fallback for the demodulator path.")
     L = C.CDLL(LIB_PATH)
     L.vdl2gpu_create.argtypes = [C.POINTER(_Config), C.POINTER(C.c_void_p)]
+    L.vdl2gpu_create_streams.argtypes = [C.POINTER(_Config), C.POINTER(_StreamLayout), C.POINTER(C.c_void_p)]
     L.vdl2gpu_destroy.argtypes = [C.c_void_p]
     L.vdl2gpu_submit.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32]
     L.vdl2gpu_submit_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]
@@ -183,12 +188,45 @@ def parse_records(region_bytes, decimated_rate):
 
 
 class Vdl2Channels:
-    """N VDL2 channels demodulated from one IQ stream on one B200."""
+    """N VDL2 channels demodulated from one IQ stream on one B200 (or from many: n_streams, from_streams)."""
 
     def __init__(self, sample_rate, oversample, sample_fmt, centerfreq, freqs, max_ppm=0.0,
                  max_chunk_bytes=1 << 20, device=-1, flags=0, n_inflight=4, n_streams=1):
         """n_streams > 1: independent-streams mode, channels [s*C, (s+1)*C) demodulate stream s; process_buf_* then take
         the S per-stream buffers back to back."""
+        n_streams = int(n_streams)
+        self._open(sample_rate, oversample, sample_fmt, centerfreq, freqs, n_streams, None, max_ppm, max_chunk_bytes, device, flags, n_inflight)
+        per = self.n_channels // n_streams if n_streams > 1 else self.n_channels
+        self.stream_of_channel = np.arange(self.n_channels, dtype=np.int64) // max(per, 1)
+
+    @classmethod
+    def from_streams(cls, sample_rate, oversample, sample_fmt, streams, max_ppm=0.0, max_chunk_bytes=1 << 20, device=-1, flags=0,
+                     n_inflight=4):
+        """Receiver farm (vdl2gpu_create_streams): `streams` is a list of (centerfreq, [freqs...]) pairs, one per receiver;
+        a receiver may carry any number of channels, none included.  Channels are numbered stream-major (stream 0's
+        first); `stream_of_channel[k]` is channel k's stream.  process_buf_* / submit / submit_device take the
+        n_streams per-stream buffers of equal length back to back."""
+        streams = list(streams)
+        if not streams:
+            raise ValueError("from_streams: at least one stream is required")
+        centres, counts, freqs = [], [], []
+        for k, st in enumerate(streams):
+            try:
+                centre, fs = st
+                fs = [int(f) for f in fs]
+            except (TypeError, ValueError):
+                raise ValueError(f"from_streams: stream {k} is not a (centerfreq, [freqs...]) pair") from None
+            centres.append(int(centre)); counts.append(len(fs)); freqs.extend(fs)
+        self = cls.__new__(cls)
+        layout = (np.asarray(counts, np.uint32), np.asarray(centres, np.uint32))
+        self._open(sample_rate, oversample, sample_fmt, centres[0], freqs, len(streams), layout, max_ppm, max_chunk_bytes, device,
+                   flags, n_inflight)
+        self.centerfreqs = layout[1]
+        self.stream_of_channel = np.repeat(np.arange(len(streams), dtype=np.int64), layout[0])
+        return self
+
+    def _open(self, sample_rate, oversample, sample_fmt, centerfreq, freqs, n_streams, layout, max_ppm, max_chunk_bytes, device,
+              flags, n_inflight):
         self.L = load_library()
         self.n_streams = int(n_streams)
         self.freqs = np.ascontiguousarray(freqs, dtype=np.uint32)
@@ -201,7 +239,12 @@ class Vdl2Channels:
         cfg.max_ppm, cfg.max_chunk_bytes, cfg.device, cfg.flags, cfg.n_inflight = max_ppm, max_chunk_bytes, device, flags, n_inflight
         cfg.n_streams = self.n_streams
         self.h = C.c_void_p()
-        _check(self.L, self.L.vdl2gpu_create(C.byref(cfg), C.byref(self.h)), "vdl2gpu_create")
+        if layout is None:
+            _check(self.L, self.L.vdl2gpu_create(C.byref(cfg), C.byref(self.h)), "vdl2gpu_create")
+        else:
+            counts, centres = layout
+            lay = _StreamLayout(self.n_streams, counts.ctypes.data_as(C.POINTER(C.c_uint32)), centres.ctypes.data_as(C.POINTER(C.c_uint32)))
+            _check(self.L, self.L.vdl2gpu_create_streams(C.byref(cfg), C.byref(lay), C.byref(self.h)), "vdl2gpu_create_streams")
         self._frames = []
         self._cb = _FRAME_CB(self._on_frame)
 

@@ -85,6 +85,9 @@ struct vdl2gpu_ctx {
 	int n_sms = 148;
 	uint32_t n_streams = 1, ch_per_stream = 0;          /* independent-streams mode: n_streams > 1, channels [s*C, (s+1)*C) on stream s */
 	bool lane_streams = false;                          /* C == 1: samples kept time-major across streams, one lane per stream in K1 */
+	bool farm = false;                                  /* receiver farm (vdl2gpu_create_streams): any channel count per stream, K1 reads the raw bytes */
+	vdl2_k1_farm k1f;                                   /* farm: per-block stream lists (d_farm) and the farm K1's tile shape */
+	uint32_t *d_farm = nullptr;
 	uint32_t raw_bytes = 0;                             /* size of each slot's raw staging buffers (allocated on the first host submit) */
 	int k1_variant = 2, k2_variant = 5, k2a_mode = 1;   /* A/B knobs (VDL2GPU_K1_VARIANT, VDL2GPU_K2_VARIANT, VDL2GPU_K2A), read at create */
 	bool use_graphs = true;
@@ -129,8 +132,8 @@ static uint32_t dphi_for(uint32_t centerfreq, uint32_t freq, uint32_t rate) {   
 	return (uint32_t)(int)(((float)centerfreq - (float)freq) / (float)rate * 256.0f * 65536.0f);
 }
 
-static void initial_state(const vdl2gpu_config &cfg, const uint32_t *freqs, uint32_t n_ch, uint32_t n_chp, uint32_t lanes, uint32_t full_warps,
-		std::vector<uint32_t> &k1, std::vector<uint32_t> &k2);
+static void initial_state(const vdl2gpu_config &cfg, const uint32_t *freqs, const uint32_t *centers, uint32_t n_ch, uint32_t n_chp, uint32_t lanes,
+		uint32_t full_warps, std::vector<uint32_t> &k1, std::vector<uint32_t> &k2);
 /* channel -> slot: the first full_warps warps hold `lanes` channels each, the others lanes - 1 */
 static inline uint32_t slot_of(uint32_t ch, uint32_t lanes, uint32_t full_warps) {
 	const uint32_t head = full_warps * lanes;
@@ -187,7 +190,7 @@ static int free_ctx(vdl2gpu_ctx *c) {
 	for(int i = 0; i < 2; i++) { cudaFree(c->d_phase2[i]); cudaFree(c->d_mag2[i]); }
 	cudaFree(c->d_k1); cudaFree(c->d_k2);
 	cudaFree(c->d_counters); cudaFree(c->d_ready); cudaFree(c->d_ring); cudaFree(c->d_pool); cudaFree(c->d_free);
-	cudaFree(c->d_ctl); cudaFree(c->d_events); cudaFree(c->d_block_trace);
+	cudaFree(c->d_ctl); cudaFree(c->d_events); cudaFree(c->d_block_trace); cudaFree(c->d_farm);
 	if(c->ev_input_ready) cudaEventDestroy(c->ev_input_ready);
 	if(c->ev_input_consumed) cudaEventDestroy(c->ev_input_consumed);
 	if(c->ev_drain) cudaEventDestroy(c->ev_drain);
@@ -201,7 +204,8 @@ static int free_ctx(vdl2gpu_ctx *c) {
 	return VDL2GPU_OK;
 }
 
-static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
+/* layout: NULL for vdl2gpu_create, the (validated) receiver-farm layout for vdl2gpu_create_streams */
+static int create_impl(const vdl2gpu_config *cfg, const vdl2gpu_stream_layout *layout, vdl2gpu_ctx *c) {
 	int ndev = 0;
 	cudaError_t e = cudaGetDeviceCount(&ndev);
 	if(e != cudaSuccess || ndev == 0) {
@@ -220,12 +224,13 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 	}
 	KL(vdl2_kernels_init_device(c->device));             /* per device: function attributes do not carry over */
 	c->cfg = *cfg;
-	c->n_streams = cfg->n_streams ? cfg->n_streams : 1u;
+	c->farm = layout != nullptr;
+	c->n_streams = c->farm ? layout->n_streams : cfg->n_streams ? cfg->n_streams : 1u;
 	c->cfg.n_streams = c->n_streams;
-	c->lane_streams = c->n_streams > 1 && c->n_streams == cfg->n_channels;     /* one stream per channel */
+	c->lane_streams = !c->farm && c->n_streams > 1 && c->n_streams == cfg->n_channels;     /* one stream per channel */
 	if(c->lane_streams) {
 		c->ch_per_stream = 1;
-	} else if(c->n_streams > 1) {
+	} else if(!c->farm && c->n_streams > 1) {
 		if(cfg->n_channels % c->n_streams != 0 || (cfg->n_channels / c->n_streams) % 32u != 0) {
 			snprintf(g_last_error, sizeof(g_last_error), "independent-streams mode needs n_channels = n_streams x C with C = 1 or a multiple of 32 (got %u channels, %u streams)",
 					cfg->n_channels, c->n_streams);
@@ -249,7 +254,7 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 		 * magnitudes from the samples (no magnitude plane, hence nothing left for K2a to do) */
 		const char *e = getenv("VDL2GPU_FUSE_PHASE");
 		const int k2v = c->k2_variant & 0xFF;
-		c->fuse_phase = (e && atoi(e) != 0) && c->k2a_mode == 1 && !(k2v >= 0 && k2v <= 4) && c->stages == 2
+		c->fuse_phase = (e && atoi(e) != 0) && !c->farm && c->k2a_mode == 1 && !(k2v >= 0 && k2v <= 4) && c->stages == 2
 			&& vdl2_k1_fuses_phase(cfg->oversample, c->ch_per_stream, (cfg->flags & VDL2GPU_FLAG_K1_SCALAR) ? 1 : 0, c->k1_variant);
 	}
 	if(cfg->flags & (VDL2GPU_FLAG_NO_GRAPH | VDL2GPU_FLAG_TRACE)) c->use_graphs = false;
@@ -267,7 +272,7 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 	 * sub-partitions, they are dealt out evenly over ALL of them: every warp holds floor or ceil of n_ch / (4 x SMs)
 	 * channels instead of 32 (27 or 28 at 16384 channels on 148 SMs), each of the two kernels launches exactly one block
 	 * per SM, every block lives for the whole kernel, and every SM looks the same to the scheduler. */
-	if(cfg->n_streams <= 1 || cfg->n_streams == cfg->n_channels) {
+	if(c->farm || cfg->n_streams <= 1 || cfg->n_streams == cfg->n_channels) {
 		const uint32_t warps_all = 4u * (uint32_t)c->n_sms;
 		if(c->n_ch > 16u * warps_all && c->n_ch <= 32u * warps_all) {
 			const char *e = getenv("VDL2GPU_BALANCE");
@@ -320,7 +325,7 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 	CU(cudaMalloc(&c->d_tab, sizeof(vdl2_tables)));
 	CU(cudaMemcpy(c->d_tab, &c->tab.t, sizeof(vdl2_tables), cudaMemcpyHostToDevice));
 	if(c->lane_streams) CU(cudaMalloc(&c->d_samples, (size_t)c->max_pairs * c->n_chp * sizeof(float2)));
-	else CU(cudaMalloc(&c->d_samples, (size_t)c->n_streams * c->max_pairs * sizeof(float2)));
+	else if(!c->farm) CU(cudaMalloc(&c->d_samples, (size_t)c->n_streams * c->max_pairs * sizeof(float2)));     /* the farm K1 reads raw bytes */
 	for(int i = 0; i < 3; i++) {
 		CU(cudaMalloc(&c->d_dec3[i], (size_t)c->max_dec * c->n_chp * sizeof(float2)));
 		CU(cudaMemset(c->d_dec3[i], 0, (size_t)c->max_dec * c->n_chp * sizeof(float2)));
@@ -343,8 +348,43 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 	CU(cudaMemset(c->d_ring, 0, (size_t)VDL2_SYNC_BUFLEN * c->n_chp * 4));
 	CU(cudaMemset(c->d_pool, 0, (size_t)c->n_slots * sizeof(vdl2_burst_slot)));
 
+	std::vector<uint32_t> centers;                      /* farm: the centre frequency of every channel's stream */
+	if(c->farm) {
+		/* per 128-slot K1 block: the streams its channels read (compacted: a stream without a channel in the block is not
+		 * listed) and every slot's column in that list.  Channels are stream-major and the slot mapping is monotone, so a
+		 * block's list comes out in ascending order and a warp holds channels of one or a few neighbouring streams. */
+		std::vector<uint32_t> stream_of(c->n_ch);
+		centers.resize(c->n_ch);
+		for(uint32_t s = 0, k = 0; s < layout->n_streams; s++)
+			for(uint32_t i = 0; i < layout->channels_per_stream[s]; i++, k++) {
+				stream_of[k] = s;
+				centers[k] = layout->centerfreqs ? layout->centerfreqs[s] : cfg->centerfreq;
+			}
+		const uint32_t blocks = (c->n_chp + K1F_BLOCK - 1) / K1F_BLOCK;
+		std::vector<uint32_t> tab((size_t)blocks * (1 + K1F_BLOCK) + c->n_chp, 0u);
+		uint32_t *col = tab.data() + (size_t)blocks * (1 + K1F_BLOCK);
+		uint32_t max_list = 1;
+		for(uint32_t ch = 0; ch < c->n_ch; ch++) {
+			const uint32_t slot = slot_of(ch, c->lanes, c->full_warps);
+			uint32_t *l = tab.data() + (size_t)(slot / K1F_BLOCK) * (1 + K1F_BLOCK);
+			if(l[0] == 0 || l[l[0]] != stream_of[ch]) { l[1 + l[0]] = stream_of[ch]; l[0]++; }
+			col[slot] = l[0] - 1;
+			max_list = std::max(max_list, l[0]);
+		}
+		if(vdl2_k1_farm_layout(cfg->oversample, cfg->sample_fmt, max_list, &c->k1f) != 0) {
+			snprintf(g_last_error, sizeof(g_last_error), "no receiver-farm K1 tile fits for oversample %u, format %u, %u streams per block",
+					cfg->oversample, cfg->sample_fmt, max_list);
+			return VDL2GPU_EINVAL;
+		}
+		CU(cudaMalloc(&c->d_farm, tab.size() * 4));
+		CU(cudaMemcpy(c->d_farm, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice));
+		c->k1f.raw = nullptr;
+		c->k1f.list = c->d_farm;
+		c->k1f.col = c->d_farm + (size_t)blocks * (1 + K1F_BLOCK);
+		c->k1f.levels = c->d_tab->levels;
+	}
 	std::vector<uint32_t> k1, k2;
-	initial_state(c->cfg, c->freqs.data(), c->n_ch, c->n_chp, c->lanes, c->full_warps, k1, k2);
+	initial_state(c->cfg, c->freqs.data(), c->farm ? centers.data() : nullptr, c->n_ch, c->n_chp, c->lanes, c->full_warps, k1, k2);
 	CU(cudaMemcpy(c->d_k1, k1.data(), k1.size() * 4, cudaMemcpyHostToDevice));
 	CU(cudaMemcpy(c->d_k2, k2.data(), k2.size() * 4, cudaMemcpyHostToDevice));
 	std::vector<int32_t> fl(c->n_slots);
@@ -370,17 +410,50 @@ static int create_impl(const vdl2gpu_config *cfg, vdl2gpu_ctx *c) {
 	return VDL2GPU_OK;
 }
 
-extern "C" int vdl2gpu_create(const vdl2gpu_config *cfg, vdl2gpu_ctx **out) {
+static int check_config(const vdl2gpu_config *cfg, vdl2gpu_ctx **out) {
 	if(!cfg || !out || !cfg->freqs || cfg->n_channels == 0 || cfg->oversample == 0 || cfg->sample_fmt > 1
 			|| cfg->sample_rate != (uint32_t)VDL2_SYMBOL_RATE * VDL2_SPS * cfg->oversample) {
 		snprintf(g_last_error, sizeof(g_last_error), "bad vdl2gpu_config (sample_rate must be 105000*oversample)");
 		return VDL2GPU_EINVAL;
 	}
+	return VDL2GPU_OK;
+}
+
+static int create_checked(const vdl2gpu_config *cfg, const vdl2gpu_stream_layout *layout, vdl2gpu_ctx **out) {
 	vdl2gpu_ctx *c = new vdl2gpu_ctx();
-	int rc = create_impl(cfg, c);
+	int rc = create_impl(cfg, layout, c);
 	if(rc != VDL2GPU_OK) { free_ctx(c); *out = nullptr; return rc; }
 	*out = c;
 	return VDL2GPU_OK;
+}
+
+extern "C" int vdl2gpu_create(const vdl2gpu_config *cfg, vdl2gpu_ctx **out) {
+	int rc = check_config(cfg, out);
+	return rc ? rc : create_checked(cfg, nullptr, out);
+}
+
+/* receiver farm: the whole layout is checked here, before any device call */
+extern "C" int vdl2gpu_create_streams(const vdl2gpu_config *cfg, const vdl2gpu_stream_layout *layout, vdl2gpu_ctx **out) {
+	int rc = check_config(cfg, out);
+	if(rc) return rc;
+#define FARM_BAD(...) do { snprintf(g_last_error, sizeof(g_last_error), "vdl2gpu_create_streams: " __VA_ARGS__); return VDL2GPU_EINVAL; } while(0)
+	if(!layout || !layout->channels_per_stream || layout->n_streams == 0) FARM_BAD("a layout with n_streams >= 1 and channels_per_stream is required");
+	if(cfg->n_streams != 0 && cfg->n_streams != layout->n_streams) FARM_BAD("cfg->n_streams (%u) must be 0 or layout->n_streams (%u)", cfg->n_streams, layout->n_streams);
+	uint64_t sum = 0;
+	for(uint32_t s = 0; s < layout->n_streams; s++) sum += layout->channels_per_stream[s];
+	if(sum != cfg->n_channels) FARM_BAD("channels_per_stream sums to %llu, n_channels is %u", (unsigned long long)sum, cfg->n_channels);
+	if(cfg->oversample != 10 && cfg->oversample != 13 && cfg->oversample != 20) FARM_BAD("oversample must be 10, 13 or 20 (got %u)", cfg->oversample);
+	if(cfg->flags & VDL2GPU_FLAG_K1_SCALAR) FARM_BAD("VDL2GPU_FLAG_K1_SCALAR is not available for receiver farms");
+	for(uint32_t s = 0, k = 0; s < layout->n_streams; s++) {
+		const int64_t centre = layout->centerfreqs ? layout->centerfreqs[s] : cfg->centerfreq;
+		for(uint32_t i = 0; i < layout->channels_per_stream[s]; i++, k++) {
+			const int64_t d = (int64_t)cfg->freqs[k] - centre;
+			if(2 * (d < 0 ? -d : d) >= (int64_t)cfg->sample_rate)
+				FARM_BAD("channel %u (%u Hz) is not within sample_rate/2 of its stream %u's centre %lld Hz", k, cfg->freqs[k], s, (long long)centre);
+		}
+	}
+#undef FARM_BAD
+	return create_checked(cfg, layout, out);
 }
 
 extern "C" int vdl2gpu_destroy(vdl2gpu_ctx *ctx) { return free_ctx(ctx); }
@@ -460,7 +533,7 @@ static void parse_region(const uint8_t *region, uint32_t out_cap, double rate, s
 static void harvest(vdl2gpu_ctx *c, chunk_slot &s) {
 	if(s.timed) {
 		static const int from[5] = { 0, 1, 3, 7, 4 }, to[5] = { 1, 2, 6, 4, 5 };   /* K0, K1 front stream; K2a middle stream; K2, K3 back stream */
-		for(int k = 0; k < 5; k++) {
+		for(int k = c->farm ? 1 : 0; k < 5; k++) {              /* a farm has no K0 */
 			float ms = 0.f;
 			if(cudaEventElapsedTime(&ms, s.tk[from[k]], s.tk[to[k]]) == cudaSuccess) { c->k_ms[k] += ms; c->k_launches[k]++; }
 		}
@@ -596,6 +669,7 @@ static int body_front(void *a) {
 	(void)pa; (void)p2; (void)p3;
 	CU(cudaMemcpyAsync(e->s->d_args, e->s->h_args, sizeof(vdl2_chunk_args), cudaMemcpyHostToDevice, c->stream));
 	const uint32_t bpp = c->cfg.sample_fmt == VDL2GPU_FMT_S16_LE ? 4u : 2u;
+	if(c->farm) { KL(vdl2_launch_k1_farm(&p1, &c->k1f, c->stream)); return 0; }      /* no K0: the farm K1 reads ca->raw */
 	if(c->lane_streams) KL(vdl2_launch_k0_lanes(nullptr, e->n_pairs, e->k0_fmt, c->d_tab->levels, reinterpret_cast<float *>(c->d_samples), c->n_streams,
 			e->n_pairs * bpp, c->n_chp, c->lanes, c->full_warps, e->s->d_args, c->stream));
 	else KL(vdl2_launch_k0(nullptr, e->n_pairs, e->k0_fmt, c->d_tab->levels, reinterpret_cast<float *>(c->d_samples), c->n_streams,
@@ -670,6 +744,11 @@ static int run_chain(vdl2gpu_ctx *c, chunk_slot &s, const void *d_raw, uint32_t 
 	if(s.timed) { CU(cudaEventRecord(s.tk[0], c->stream)); if(graph) CU(cudaEventRecord(s.tk[1], c->stream)); }
 	if(graph) {
 		CU(cudaGraphLaunch(s.g_front[gk], c->stream));
+	} else if(c->farm) {
+		vdl2_k1_farm f = c->k1f;
+		f.raw = d_raw;
+		if(s.timed) CU(cudaEventRecord(s.tk[1], c->stream));
+		KL(vdl2_launch_k1_farm(&p1, &f, c->stream));
 	} else {
 		if(c->lane_streams) KL(vdl2_launch_k0_lanes(d_raw, n_pairs, k0_fmt, c->d_tab->levels, reinterpret_cast<float *>(c->d_samples), c->n_streams,
 				n_pairs * bpp, c->n_chp, c->lanes, c->full_warps, nullptr, c->stream));
@@ -720,7 +799,7 @@ static int run_chain(vdl2gpu_ctx *c, chunk_slot &s, const void *d_raw, uint32_t 
 	c->stats.chunks_submitted++;
 	c->stats.iq_samples += n_pairs;
 	c->stats.dec_samples += s.n_dec;
-	c->stats.kernel_launches += (n_pairs ? 2 : 0) + (c->fuse_phase ? 0 : 1) + (s.n_dec ? 1 : 0) + 2;
+	c->stats.kernel_launches += (n_pairs ? (c->farm ? 1 : 2) : 0) + (c->fuse_phase ? 0 : 1) + (s.n_dec ? 1 : 0) + 2;
 	return VDL2GPU_OK;
 }
 
@@ -748,7 +827,7 @@ extern "C" int vdl2gpu_submit(vdl2gpu_ctx *c, const void *iq, uint32_t len) {
 
 extern "C" int vdl2gpu_submit_planar_s16(vdl2gpu_ctx *c, const int16_t *xi, const int16_t *xq, uint32_t n_pairs) {
 	if(!c || ((!xi || !xq) && n_pairs)) return VDL2GPU_EINVAL;
-	if(c->cfg.sample_fmt != VDL2GPU_FMT_S16_LE || c->n_streams != 1) return VDL2GPU_EINVAL;
+	if(c->cfg.sample_fmt != VDL2GPU_FMT_S16_LE || c->n_streams != 1 || c->farm) return VDL2GPU_EINVAL;
 	if(n_pairs == 0) return VDL2GPU_OK;
 	if((uint64_t)n_pairs * 4u > c->cfg.max_chunk_bytes) return VDL2GPU_ETOOBIG;
 	CU(cudaSetDevice(c->device));
@@ -1145,16 +1224,18 @@ extern "C" size_t vdl2gpu_stage_device_bytes(uint32_t n_channels, uint32_t max_d
 extern "C" uint32_t vdl2gpu_stage_row_stride(uint32_t n_channels) { return (n_channels + 31u) & ~31u; }
 
 /* initial per-channel state: vdl2_channel_init + demod_reset (src/demod.c:205-220,379-392), process_samples locals
- * (src/demod.c:289-298); shared by the batch context and the stage stubs */
-static void initial_state(const vdl2gpu_config &cfg, const uint32_t *freqs, uint32_t n_ch, uint32_t n_chp, uint32_t lanes, uint32_t full_warps,
-		std::vector<uint32_t> &k1, std::vector<uint32_t> &k2) {
+ * (src/demod.c:289-298); shared by the batch context and the stage stubs.  centers: the centre frequency of every
+ * channel's stream (receiver farm), NULL = cfg.centerfreq for all */
+static void initial_state(const vdl2gpu_config &cfg, const uint32_t *freqs, const uint32_t *centers, uint32_t n_ch, uint32_t n_chp, uint32_t lanes,
+		uint32_t full_warps, std::vector<uint32_t> &k1, std::vector<uint32_t> &k2) {
 	k1.assign((size_t)K1_NFIELDS * n_chp, 0u); k2.assign((size_t)K2_NFIELDS * n_chp, 0u);
 	auto fbits = [](float f) { uint32_t u; memcpy(&u, &f, 4); return u; };
 	for(uint32_t chan = 0; chan < n_ch; chan++) {
 		const uint32_t ch = slot_of(chan, lanes, full_warps);          /* index into the per-channel planes */
 		/* a channel on the centre frequency skips the mixer in the reference (src/demod.c:312); with a zero
 		 * phase step the table gives cos = 1, sin = 0 and the products are exact, so no branch is needed */
-		k1[(size_t)K1_DPHI * n_chp + ch] = (cfg.centerfreq != freqs[chan]) ? dphi_for(cfg.centerfreq, freqs[chan], cfg.sample_rate) : 0u;
+		const uint32_t centre = centers ? centers[chan] : cfg.centerfreq;
+		k1[(size_t)K1_DPHI * n_chp + ch] = (centre != freqs[chan]) ? dphi_for(centre, freqs[chan], cfg.sample_rate) : 0u;
 		k2[(size_t)K2_MAG_NF * n_chp + ch] = fbits(2.0f);
 		k2[(size_t)K2_PHERR1 * n_chp + ch] = fbits(1000.f);
 		k2[(size_t)K2_PHERR2 * n_chp + ch] = fbits(1000.f);
@@ -1195,7 +1276,7 @@ extern "C" int vdl2gpu_stage_create(const vdl2gpu_config *cfg, uint32_t max_dec,
 	st->d_ready = reinterpret_cast<uint32_t *>(b + L.ready); st->d_ctl = reinterpret_cast<vdl2_queue_ctl *>(b + L.ctl);
 	st->d_events = b + L.events;
 	std::vector<uint32_t> k1, k2;
-	initial_state(st->cfg, st->freqs.data(), st->n_ch, st->n_chp, 32u, 0xFFFFFFFFu, k1, k2);
+	initial_state(st->cfg, st->freqs.data(), nullptr, st->n_ch, st->n_chp, 32u, 0xFFFFFFFFu, k1, k2);
 	std::vector<int32_t> fl(st->n_slots);
 	for(uint32_t i = 0; i < st->n_slots; i++) fl[i] = (int32_t)i;
 	vdl2_queue_ctl ctl;

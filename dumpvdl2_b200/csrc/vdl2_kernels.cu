@@ -46,6 +46,14 @@ __device__ __forceinline__ bool vdl2_slot_channel(uint32_t slot, uint32_t lanes,
 /* ------------------------------------------------------------------------------------------------
  * K0: sample conversion.  Output: float2 {re, im} per complex sample (src/demod.c:339-365).
  * ---------------------------------------------------------------------------------------------- */
+/* one interleaved complex sample -> {re, im}; every kernel that reads raw input converts through these two */
+__device__ __forceinline__ float2 vdl2_iq_u8(uchar2 v, const float *__restrict__ levels) {      /* src/demod.c:343-345, table :349-354 */
+	return make_float2(__ldg(&levels[v.x]), __ldg(&levels[v.y]));
+}
+__device__ __forceinline__ float2 vdl2_iq_s16(short2 v) {                                        /* src/demod.c:361-363 */
+	return make_float2(__fdiv_rn((float)v.x, 32768.0f), __fdiv_rn((float)v.y, 32768.0f));
+}
+
 __global__ void __launch_bounds__(256) k0_convert(const uint8_t *__restrict__ raw0, uint32_t n_pairs_p, uint32_t fmt,
 		const float *__restrict__ levels, float2 *__restrict__ out0, uint32_t raw_stride, uint32_t out_stride,
 		const vdl2_chunk_args *__restrict__ ca) {
@@ -54,24 +62,20 @@ __global__ void __launch_bounds__(256) k0_convert(const uint8_t *__restrict__ ra
 	float2 *out = out0 + (size_t)blockIdx.y * out_stride;
 	uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
 	if(i >= n_pairs) return;
-	float re, im;
-	if(fmt == 0) {                                       /* src/demod.c:343-345, table from :349-354 */
-		uchar2 v = reinterpret_cast<const uchar2 *>(raw)[i];
-		re = __ldg(&levels[v.x]);
-		im = __ldg(&levels[v.y]);
-	} else if(fmt == 1) {                                /* src/demod.c:361-363 */
-		short2 v = reinterpret_cast<const short2 *>(raw)[i];
-		re = __fdiv_rn((float)v.x, 32768.0f);
-		im = __fdiv_rn((float)v.y, 32768.0f);
+	float2 v;
+	if(fmt == 0) {
+		v = vdl2_iq_u8(reinterpret_cast<const uchar2 *>(raw)[i], levels);
+	} else if(fmt == 1) {
+		v = vdl2_iq_s16(reinterpret_cast<const short2 *>(raw)[i]);
 	} else {
 		/* planar cs16: n_pairs I values followed by n_pairs Q values, the shape the SDRplay APIs deliver
 		 * (src/sdrplay.c:72, src/sdrplay3.c callbacks); same arithmetic as the interleaved case, the
 		 * host-side interleave loop of src/sdrplay.c:95-121 is not needed */
 		const short *pl = reinterpret_cast<const short *>(raw);
-		re = __fdiv_rn((float)pl[i], 32768.0f);
-		im = __fdiv_rn((float)pl[n_pairs + i], 32768.0f);
+		v.x = __fdiv_rn((float)pl[i], 32768.0f);
+		v.y = __fdiv_rn((float)pl[n_pairs + i], 32768.0f);
 	}
-	out[i] = make_float2(re, im);
+	out[i] = v;
 }
 
 /* K0 for the one-stream-per-channel layout: raw[s][i] -> out[i][s] float2 {re, im}, i.e. TIME-major across streams, so
@@ -87,18 +91,13 @@ __global__ void __launch_bounds__(1024) k0_convert_lanes(const uint8_t *__restri
 	const uint32_t i_in = blockIdx.x * 32u + tx;
 	uint32_t s_in;                                    /* stream = channel that lives in column (slot) blockIdx.y * 32 + ty */
 	const bool have = vdl2_slot_channel(blockIdx.y * 32u + ty, lanes, full_warps, n_streams, s_in);
-	float re = 0.f, im = 0.f;
+	float2 v = make_float2(0.f, 0.f);
 	if(have && i_in < n_pairs) {
 		const uint8_t *r = raw + (size_t)s_in * raw_stride;
-		if(fmt == 0) {
-			uchar2 v = reinterpret_cast<const uchar2 *>(r)[i_in];
-			re = __ldg(&levels[v.x]); im = __ldg(&levels[v.y]);
-		} else {
-			short2 v = reinterpret_cast<const short2 *>(r)[i_in];
-			re = __fdiv_rn((float)v.x, 32768.0f); im = __fdiv_rn((float)v.y, 32768.0f);
-		}
+		if(fmt == 0) v = vdl2_iq_u8(reinterpret_cast<const uchar2 *>(r)[i_in], levels);
+		else v = vdl2_iq_s16(reinterpret_cast<const short2 *>(r)[i_in]);
 	}
-	tile[ty][tx] = make_float2(re, im);
+	tile[ty][tx] = v;
 	__syncthreads();
 	const uint32_t i_out = blockIdx.x * 32u + ty, s_out = blockIdx.y * 32u + tx;
 	if(i_out < n_pairs && s_out < out_stride) out[(size_t)i_out * out_stride + s_out] = tile[tx][ty];
@@ -604,6 +603,188 @@ __global__ void __launch_bounds__(K1L_BLOCK) k1_mix_iir_decimate_lanes(vdl2_k1_p
 		}
 		k1_store_state(p, ch, f2_lo(x1), f2_lo(x2), f2_hi(x1), f2_hi(x2), f2_lo(y1), f2_lo(y2), f2_hi(y1), f2_hi(y2), phi);
 	}
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * K1, receiver farm (vdl2gpu_create_streams): many raw IQ streams, each with its own centre frequency and any number of
+ * channels, the channels stream-major in the slots.  A 128-slot block reads only the streams its channels belong to (the
+ * host lists them per block: vdl2_k1_farm.list, .col).  Per tile of R = groups x OS rows, thread j of the block fetches
+ * listed stream j's raw bytes (cu8 or cs16, straight from the caller's buffer) with one cp.async.bulk into a double-
+ * buffered raw tile, arriving on the tile's mbarrier with its own byte count.  The block then converts the tile once per
+ * stream-sample (vdl2_iq_u8 / vdl2_iq_s16, the arithmetic of K0) into a float2 tile [R][row], and lane `slot` reads
+ * column col[slot] of each row: the lanes of a warp hold channels of one or a few neighbouring streams, so a row read is
+ * a broadcast or a single wavefront.  No K0 launch and no float sample plane.  The filter arithmetic and the eight-copy
+ * NCO table are those of the lanes kernel; head and tail samples (outside whole tiles) are converted per lane from the
+ * raw bytes.
+ *
+ * A stream's segment of tile t starts at s * n_pairs * bpp + (head + t R) * bpp, not 16-byte aligned in general (the
+ * caller chooses len and the buffer): the copy fetches from the 16-byte boundary at or below it, rounds the size up to
+ * 16 bytes and the conversion skips the `off` leading bytes.  The extra bytes lie in 16-byte granules that also hold
+ * bytes of the segment, so they are always mapped.
+ *
+ * Shared memory (dynamic, k1f_layout): NCO table 257 x 8 x 16 B = 32,896 B; float tile R x row x 8 B with row = the
+ * longest list of any block, made odd so that the conversion's column writes (32 rows of one stream) avoid bank
+ * conflicts; raw tiles 2 x n x W with W = roundup16(15 + R x bpp); two mbarriers; the block's list (4 B) and window
+ * offsets (2 x 1 B) per stream.  The host takes the longest tile (at most 640 samples, like the packed kernel) that
+ * keeps the total within K1F_SMEM_MAX = 90 KB, so that one farm block fits beside one K2 block (120,848 B) in the
+ * 228 KB of an SM, as the packed K1 does.  Worst case, 128 streams in a block, cs16: at OS 10 and 20 R = 20 ->
+ * 32,896 + 20 x 129 x 8 + 2 x 128 x 96 + 16 + 768 = 78,896 B; at OS 13 R = 13 -> 32,896 + 13,424 (13 x 129 x 8 rounded to
+ * 16) + 2 x 128 x 80 + 16 + 768 = 67,584 B (R = 26 would need 93,280 B).
+ * ---------------------------------------------------------------------------------------------- */
+#define K1F_SMEM_MAX (90 * 1024)
+#define K1F_LUT_BYTES (257 * 8 * 16)
+#define K1F_MAX_TILE 640
+
+struct k1f_layout {
+	uint32_t row, win, ft, raw, bar, list, off, total;       /* float2 per tile row, bytes per raw window, byte offsets */
+	__host__ __device__ k1f_layout(uint32_t rows, uint32_t max_list, uint32_t bpp) {
+		row = max_list | 1u;
+		win = (15u + rows * bpp + 15u) & ~15u;
+		ft = K1F_LUT_BYTES;
+		raw = ft + ((rows * row * 8u + 15u) & ~15u);
+		bar = raw + 2u * max_list * win;
+		list = bar + 16u;
+		off = list + 4u * max_list;
+		total = off + 2u * max_list;
+	}
+};
+
+template<int OS, bool SYM>
+__global__ void __launch_bounds__(K1F_BLOCK) k1_mix_iir_decimate_farm(vdl2_k1_params p, vdl2_k1_farm f) {
+	constexpr int LA = 10, MA = 5;
+	constexpr int NLUT = 8;
+	extern __shared__ __align__(128) unsigned char k1f_smem[];
+	const uint32_t tid = threadIdx.x, warp = tid >> 5, lane = tid & 31u;
+	const int trace_k = tid == 0 ? vdl2_trace_begin(p.trace_blocks, 1) : -1;
+	const uint32_t ch = blockIdx.x * K1F_BLOCK + tid;
+	uint32_t chan;
+	const bool active = vdl2_slot_channel(ch, p.lanes, p.full_warps, p.n_ch, chan);
+	const uint32_t n_pairs = p.ca ? p.ca->n_pairs : p.n_pairs, cnt0 = p.ca ? p.ca->cnt0 : p.cnt0;
+	const uint8_t *raw = static_cast<const uint8_t *>(p.ca ? p.ca->raw : f.raw);
+	const bool s16 = f.fmt == 1u;
+	const uint32_t bpp = s16 ? 4u : 2u;
+	const size_t stride = (size_t)n_pairs * bpp;                  /* bytes between consecutive streams */
+	const uint32_t *blist = f.list + (size_t)blockIdx.x * (1u + K1F_BLOCK);
+	const uint32_t n_list = blist[0], G = f.groups, R = G * OS;
+	const k1f_layout lay(R, f.max_list, bpp);
+	float4 *s_lut = reinterpret_cast<float4 *>(k1f_smem);
+	float2 *s_ft = reinterpret_cast<float2 *>(k1f_smem + lay.ft);
+	uint8_t *s_raw = k1f_smem + lay.raw;
+	uint64_t *s_bar = reinterpret_cast<uint64_t *>(k1f_smem + lay.bar);
+	uint32_t *s_list = reinterpret_cast<uint32_t *>(k1f_smem + lay.list);
+	uint8_t *s_off = k1f_smem + lay.off;                          /* [2][max_list]: where the segment starts in its window */
+	for(uint32_t i = tid; i < 257 * NLUT; i += K1F_BLOCK) s_lut[i] = p.lut[i / NLUT];
+	const float4 *lut = s_lut + (tid & (NLUT - 1));
+	const uint32_t lane_bytes = (tid & (NLUT - 1)) * 16u;
+	if(tid < n_list) s_list[tid] = blist[1 + tid];
+	if(tid == 0 && n_list) { mbar_init(&s_bar[0], n_list); mbar_init(&s_bar[1], n_list); mbar_fence_init(); }
+	float xr1 = 0, xr2 = 0, xi1 = 0, xi2 = 0, yr1 = 0, yr2 = 0, yi1 = 0, yi2 = 0;
+	uint32_t phi = 0, dphi = 0;
+	if(active) k1_load_state(p, ch, xr1, xr2, xi1, xi2, yr1, yr2, yi1, yi2, phi, dphi);
+	u64 x1 = f2_pack(xr1, xi1), x2 = f2_pack(xr2, xi2), y1 = f2_pack(yr1, yi1), y2 = f2_pack(yr2, yi2);
+	k1_packed_consts c;
+	c.ONE = f2_pack(p.one, p.one); c.SGN = f2_pack(p.neg_one, p.one);
+	c.A0 = f2_pack(p.a0, p.a0); c.A1 = f2_pack(p.a1, p.a1); c.A2 = f2_pack(p.a2, p.a2);
+	c.B1 = f2_pack(p.b1, p.b1); c.B2 = f2_pack(p.b2, p.b2); c.TWO = f2_pack(p.two, p.two);
+	c.one = p.one; c.neg_one = p.neg_one;
+	const uint32_t col = active ? f.col[ch] : 0u;
+	__syncthreads();
+	if(n_list == 0) { if(tid == 0) vdl2_trace_end(p.trace_blocks, trace_k); return; }      /* no channel in this block */
+	const uint8_t *mine = raw + (size_t)s_list[col] * stride;     /* this lane's stream (head and tail samples) */
+	auto sample_at = [&](uint32_t i) -> float2 {
+		const uint8_t *b = mine + (size_t)i * bpp;
+		return s16 ? vdl2_iq_s16(*reinterpret_cast<const short2 *>(b)) : vdl2_iq_u8(*reinterpret_cast<const uchar2 *>(b), f.levels);
+	};
+
+	uint32_t cnt = cnt0, m = 0, pos = 0;
+	const uint32_t head = min(n_pairs, (OS - cnt0 % OS) % OS);
+	if(active) {
+		for(; pos < head; pos++) {
+			u64 y0 = k1_packed_step(sample_at(pos), lut[((phi >> 16) & 0xFFu) * NLUT], phi, dphi, x1, x2, y1, y2, c);
+			if(++cnt == OS) { cnt = 0; p.dec[(size_t)m * p.n_chp + ch] = make_float2(f2_lo(y0), f2_hi(y0)); m++; }
+		}
+	}
+	pos = head;
+	m = (cnt0 + head) / OS;
+	cnt = (cnt0 + head) % OS;
+	u64 P1 = f2_mul(c.A0, x1), P2 = f2_mul(c.A0, x2);
+	const uint32_t n_groups = (n_pairs - pos) / OS;
+	const uint32_t n_tiles = (n_groups + G - 1) / G;
+	/* thread j < n_list: stream j's segment of tile t into raw buffer `buf`, one bulk copy, one arrival on the buffer's barrier */
+	auto request = [&](uint32_t t, uint32_t buf) {
+		const uint32_t rows = min(G, n_groups - t * G) * OS;
+		const uint8_t *src = raw + (size_t)s_list[tid] * stride + (size_t)(head + t * R) * bpp;
+		const uint32_t off = (uint32_t)(reinterpret_cast<uintptr_t>(src) & 15u);
+		s_off[buf * f.max_list + tid] = (uint8_t)off;
+		tma_load_tile(s_raw + (size_t)(buf * f.max_list + tid) * lay.win, src - off, (off + rows * bpp + 15u) & ~15u, &s_bar[buf]);
+	};
+	if(tid < n_list)
+		for(uint32_t t = 0; t < 2 && t < n_tiles; t++) request(t, t);
+	for(uint32_t g0 = 0, tile = 0; g0 < n_groups; g0 += G, tile++) {
+		const uint32_t ng = min(G, n_groups - g0), rows = ng * OS, buf = tile & 1u;
+		mbar_wait(&s_bar[buf], (tile >> 1) & 1u);
+		/* conversion, once per stream-sample: warp w takes streams w, w + 4, ..., its lanes consecutive rows */
+		for(uint32_t j = warp; j < n_list; j += K1F_BLOCK / 32) {
+			const uint8_t *w = s_raw + (size_t)(buf * f.max_list + j) * lay.win + s_off[buf * f.max_list + j];
+			for(uint32_t r = lane; r < rows; r += 32)
+				s_ft[r * lay.row + j] = s16 ? vdl2_iq_s16(*reinterpret_cast<const short2 *>(w + r * 4u))
+				                            : vdl2_iq_u8(*reinterpret_cast<const uchar2 *>(w + r * 2u), f.levels);
+		}
+		__syncthreads();                                           /* the float tile is complete, raw buffer `buf` is free */
+		if(tid < n_list && tile + 2 < n_tiles) request(tile + 2, buf);
+		if(active) {
+			for(uint32_t g = 0; g < ng; g++) {
+				const float2 *sp = s_ft + (size_t)g * OS * lay.row + col;
+				u64 y0 = 0;
+				float2 S[OS];
+				float4 E[OS];
+				float FR[OS];
+				u64 X0[OS];
+#pragma unroll
+				for(int k = -LA; k < OS; k++) {
+					const int kl = k + LA, km = k + MA;
+					if(kl < OS) {
+						const uint32_t ph = phi + (uint32_t)kl * dphi;
+						E[kl] = k1_lut_entry<NLUT>(s_lut, ph, lane_bytes);
+						FR[kl] = (float)(ph & 0xFFFFu);
+						S[kl] = sp[kl * lay.row];
+					}
+					if(km >= 0 && km < OS) {
+						const u64 CS = f2_fma(f2_mul(f2_pack(E[km].z, E[km].w), f2_pack(FR[km], FR[km])), c.ONE, f2_pack(E[km].x, E[km].y));
+						X0[km] = k1_mix(S[km], CS, c);
+					}
+					if(k >= 0) {
+						const u64 x0 = X0[k];
+						u64 r;
+						if(SYM) {
+							const u64 P0 = f2_mul(c.A0, x0);
+							r = f2_fma(P0, c.ONE, f2_fma(P1, c.TWO, P2));
+							P2 = P1; P1 = P0;
+						} else {
+							const u64 t = f2_fma(f2_mul(c.A1, x1), c.ONE, f2_mul(c.A2, x2));
+							r = f2_fma(f2_mul(c.A0, x0), c.ONE, t);
+						}
+						const u64 u = f2_fma(f2_mul(c.B1, y1), c.ONE, f2_mul(c.B2, y2));
+						y0 = f2_fma(r, c.ONE, u);
+						x2 = x1; x1 = x0; y2 = y1; y1 = y0;
+					}
+				}
+				phi += (uint32_t)OS * dphi;
+				p.dec[(size_t)(m + g) * p.n_chp + ch] = make_float2(f2_lo(y0), f2_hi(y0));
+			}
+		}
+		m += ng;
+		pos += rows;
+		__syncthreads();                                           /* every warp is done with the float tile */
+	}
+	if(active) {
+		for(; pos < n_pairs; pos++) {
+			u64 y0 = k1_packed_step(sample_at(pos), lut[((phi >> 16) & 0xFFu) * NLUT], phi, dphi, x1, x2, y1, y2, c);
+			if(++cnt == OS) { cnt = 0; p.dec[(size_t)m * p.n_chp + ch] = make_float2(f2_lo(y0), f2_hi(y0)); m++; }
+		}
+		k1_store_state(p, ch, f2_lo(x1), f2_lo(x2), f2_hi(x1), f2_hi(x2), f2_lo(y1), f2_lo(y2), f2_hi(y1), f2_hi(y2), phi);
+	}
+	if(tid == 0) vdl2_trace_end(p.trace_blocks, trace_k);
 }
 
 /* ------------------------------------------------------------------------------------------------
@@ -1181,6 +1362,10 @@ extern "C" int vdl2_kernels_init_device(int device) {
 		cudaFuncSetAttribute(k1_mix_iir_decimate_lanes<20, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1L_SMEM_BYTES);
 		cudaFuncSetAttribute(k1_mix_iir_decimate_lanes<10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1L_SMEM_BYTES);
 		cudaFuncSetAttribute(k1_mix_iir_decimate_lanes<10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1L_SMEM_BYTES);
+#define K1F_SETUP(OS, SYM) do { vdl2_set_carveout(k1_mix_iir_decimate_farm<OS, SYM>, pct); \
+		cudaFuncSetAttribute(k1_mix_iir_decimate_farm<OS, SYM>, cudaFuncAttributeMaxDynamicSharedMemorySize, K1F_SMEM_MAX); } while(0)
+		K1F_SETUP(20, true); K1F_SETUP(20, false); K1F_SETUP(10, true); K1F_SETUP(10, false); K1F_SETUP(13, true); K1F_SETUP(13, false);
+#undef K1F_SETUP
 		vdl2_set_carveout(k2a_phase_mag<true>, pct);
 		vdl2_set_carveout(k2a_phase_mag_warps<true>, pct);
 		vdl2_set_carveout(k2a_phase_mag_warps<false>, pct);
@@ -1262,6 +1447,30 @@ extern "C" int vdl2_launch_k1(const vdl2_k1_params *p, int force_scalar, int var
 		const uint32_t blocks = (p->n_chp + K1_BLOCK1 - 1) / K1_BLOCK1;
 		k1_mix_iir_decimate_scalar<K1_BLOCK1><<<blocks, K1_BLOCK1, 0, st>>>(*p);
 	}
+	return (int)cudaGetLastError();
+}
+
+extern "C" int vdl2_k1_farm_layout(uint32_t oversample, uint32_t fmt, uint32_t max_list, vdl2_k1_farm *f) {
+	if((oversample != 10 && oversample != 13 && oversample != 20) || fmt > 1u || max_list == 0 || max_list > K1F_BLOCK) return (int)cudaErrorInvalidValue;
+	const uint32_t bpp = fmt == 1u ? 4u : 2u;
+	for(uint32_t g = K1F_MAX_TILE / oversample; g >= 1; g--) {
+		const k1f_layout lay(g * oversample, max_list, bpp);
+		if(lay.total <= K1F_SMEM_MAX) { f->groups = g; f->max_list = max_list; f->fmt = fmt; f->smem_bytes = lay.total; return 0; }
+	}
+	return (int)cudaErrorInvalidValue;
+}
+
+extern "C" int vdl2_launch_k1_farm(const vdl2_k1_params *p, const vdl2_k1_farm *f, cudaStream_t st) {
+	if(p->n_pairs == 0 || p->n_ch == 0) return 0;
+	const bool sym = (p->a1 == 2.0f * p->a0) && (p->a2 == p->a0);
+	const uint32_t blocks = (p->n_chp + K1F_BLOCK - 1) / K1F_BLOCK;
+#define K1F_GO(OS) do { if(sym) k1_mix_iir_decimate_farm<OS, true><<<blocks, K1F_BLOCK, f->smem_bytes, st>>>(*p, *f); \
+		else k1_mix_iir_decimate_farm<OS, false><<<blocks, K1F_BLOCK, f->smem_bytes, st>>>(*p, *f); } while(0)
+	if(p->oversample == 20) K1F_GO(20);
+	else if(p->oversample == 10) K1F_GO(10);
+	else if(p->oversample == 13) K1F_GO(13);
+	else return (int)cudaErrorInvalidValue;
+#undef K1F_GO
 	return (int)cudaGetLastError();
 }
 

@@ -58,6 +58,20 @@ typedef struct {
 	uint32_t prev_n_dec;         /* overridden by ca->prev_n_dec */
 } vdl2_k1_params;
 
+/* receiver farm (vdl2gpu_create_streams): many raw streams, each with its own channels; K1 reads the raw bytes itself */
+typedef struct {
+	const void *raw;             /* stream s at raw + s * n_pairs * bpp bytes (overridden by ca->raw) */
+	const uint32_t *list;        /* [blocks][1 + K1F_BLOCK]: per 128-slot block the number of streams its channels read, then
+	                              * those streams in ascending order */
+	const uint32_t *col;         /* [n_chp]: a slot's index into its block's stream list */
+	const float *levels;         /* cu8 level table (src/demod.c:349-354) */
+	uint32_t fmt;                /* VDL2GPU_FMT_U8 / VDL2GPU_FMT_S16_LE */
+	uint32_t groups;             /* decimation groups per staged tile */
+	uint32_t max_list;           /* largest stream list of any block (the row length of the staged tile) */
+	uint32_t smem_bytes;         /* dynamic shared memory of a block, vdl2_k1_farm_smem_bytes */
+} vdl2_k1_farm;
+#define K1F_BLOCK 128
+
 typedef struct {
 	const float2 *dec;
 	float *phase;                /* [160 + n_dec][n_chp]: rows 0..159 = last 160 phases of the previous chunks */
@@ -123,6 +137,10 @@ int vdl2_launch_k0(const void *raw, uint32_t n_pairs, uint32_t fmt, const float 
 int vdl2_launch_k0_lanes(const void *raw, uint32_t n_pairs, uint32_t fmt, const float *levels, float *out2, uint32_t n_streams,
 		uint32_t raw_stride, uint32_t out_stride, uint32_t lanes, uint32_t full_warps, const vdl2_chunk_args *ca, cudaStream_t st);
 int vdl2_launch_k1(const vdl2_k1_params *p, int force_scalar, int variant, cudaStream_t st);
+/* receiver farm: shared-memory layout of k1_mix_iir_decimate_farm for these shapes (f->groups, f->smem_bytes are set);
+ * returns 0 or cudaErrorInvalidValue when even one group per tile does not fit the block's budget */
+int vdl2_k1_farm_layout(uint32_t oversample, uint32_t fmt, uint32_t max_list, vdl2_k1_farm *f);
+int vdl2_launch_k1_farm(const vdl2_k1_params *p, const vdl2_k1_farm *f, cudaStream_t st);
 /* whether vdl2_launch_k1 with these arguments runs a kernel that honours p->phase (the pipelined packed kernel with
  * 128-channel blocks); everything else leaves the phase plane to K2a */
 int vdl2_k1_fuses_phase(uint32_t oversample, uint32_t ch_per_stream, int force_scalar, int variant);

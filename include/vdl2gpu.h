@@ -10,7 +10,8 @@
  *
  * Two front doors (INTEGRATION.md shows the reference-side binding for both):
  *
- *  (1) batch API (this file): one context = one IQ stream fanned out to N channels.  It replaces, as a
+ *  (1) batch API (this file): one context = one IQ stream fanned out to N channels, or many streams
+ *      (n_streams, vdl2gpu_create_streams) each with its own channels.  It replaces, as a
  *      unit, what the reference spreads over
  *        process_buf_uchar/process_buf_short   (src/demod.c:339-365)    -> vdl2gpu_submit
  *        N x process_samples threads + barriers (src/demod.c:288-337)   -> kernels K0-K3 on a stream
@@ -125,10 +126,25 @@ typedef struct {
 
 typedef struct vdl2gpu_ctx vdl2gpu_ctx;
 
+/* Receiver farm: n_streams IQ streams, each from its own receiver with its own centre frequency, each carrying any number
+ * of channels (0 allowed).  cfg->freqs lists the channels stream-major (stream 0's first), so channel k demodulates the
+ * stream it falls into by the running sum of channels_per_stream.  Everything after create works as with
+ * cfg->n_streams = S: submit / submit_device take S buffers of `len` bytes back to back, frames carry the channel index
+ * into cfg->freqs and its frequency.  Rules: cfg->n_streams is 0 or n_streams; counts sum to cfg->n_channels; every
+ * channel lies less than sample_rate / 2 from its stream's centre; oversample 10, 13 or 20; VDL2GPU_FMT_U8 or
+ * VDL2GPU_FMT_S16_LE; no VDL2GPU_FLAG_K1_SCALAR.  A layout that breaks one returns VDL2GPU_EINVAL before any device
+ * call. */
+typedef struct {
+	uint32_t n_streams;
+	const uint32_t *channels_per_stream; /* n_streams counts (0 allowed), sum == cfg->n_channels */
+	const uint32_t *centerfreqs;         /* n_streams centre frequencies in Hz; NULL = cfg->centerfreq for every stream */
+} vdl2gpu_stream_layout;
+
 /* ---- life cycle ---- */
 int vdl2gpu_abi_version(void);
 int vdl2gpu_device_count(void);
 int vdl2gpu_create(const vdl2gpu_config *cfg, vdl2gpu_ctx **out);
+int vdl2gpu_create_streams(const vdl2gpu_config *cfg, const vdl2gpu_stream_layout *layout, vdl2gpu_ctx **out);
 int vdl2gpu_destroy(vdl2gpu_ctx *ctx);
 const char *vdl2gpu_strerror(int code);
 const char *vdl2gpu_last_error(void);
@@ -218,7 +234,7 @@ int vdl2gpu_read_dec(vdl2gpu_ctx *ctx, float *out, size_t cap_floats, uint32_t *
 int vdl2gpu_read_events(vdl2gpu_ctx *ctx, vdl2gpu_event *out, uint32_t cap);
 /* device time (ms) spent in each kernel for the chunks completed so far, measured with CUDA events on
  * the library's streams when timing was enabled with vdl2gpu_enable_timing(ctx, 1).
- * Order: K0, K1, K2a, K2 (+history copy), K3 (+finish). */
+ * Order: K0, K1, K2a, K2 (+history copy), K3 (+finish).  A receiver farm has no K0 (0 launches). */
 int vdl2gpu_enable_timing(vdl2gpu_ctx *ctx, int on);
 int vdl2gpu_get_kernel_ms(vdl2gpu_ctx *ctx, double ms[5], uint64_t launches[5]);
 /* stage boundaries of the timed chunks harvested so far, 8 floats per chunk: chunk number, then ms since
